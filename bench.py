@@ -17,6 +17,10 @@ through the host-buffer entry (pinned uint8 frames H2D and the result records D2
 timed region).  `roofline` is for the dominant kernel, the grouped 7x7 128->128 conv launch.
 `--impl reference` times the CPU restatement of the reference path (oracle/, torch-CPU conv +
 NumPy/SciPy post-process; Chainer itself is not installable offline) on the host cores.
+
+`--dump-outputs DIR` writes what the timed path returned in its last step (the person records of one batch; poses and
+scores with --impl reference) as DIR/<name>.npy in float64.  Inputs and weights are seeded, so two builds run with the
+same arguments can be compared output for output.
 """
 import argparse
 import importlib
@@ -170,6 +174,10 @@ def run_reference(args):
         poses, scores = cpu_reference_step(weights, imgs[i % 2], paf_lo, heat_lo)
     dt = time.perf_counter() - t0
     assert len(scores) == 8
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "poses.npy"), np.asarray(poses, np.float64))
+        np.save(os.path.join(args.dump_outputs, "scores.npy"), np.asarray(scores, np.float64))
     value = args.steps / dt
     sample = ("1 frame per step (the reference is batch-1), %d steps, %d torch threads (fastest of 16/32/64/all on a "
               "%d-core host)" % (args.steps, cores, os.cpu_count()))
@@ -186,6 +194,20 @@ def run_reference(args):
         "cpu_baseline": {"value": value, "unit": "frames/s", "cores": cores, "kind": "port", "sample": sample},
         "e2e": {"value": value, "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }))
+
+
+def dump_records(out_dir, hdr, per):
+    """The person records of one batch as float64 .npy files: per-image header fields, and per-person fields with the
+    slots past each image's n_persons zeroed (the device leaves them unwritten)."""
+    os.makedirs(out_dir, exist_ok=True)
+    used = np.arange(per.shape[1])[None, :] < hdr["n_persons"][:, None]
+    arrays = {"n_peaks": hdr["n_peaks"], "n_persons": hdr["n_persons"], "status": hdr["status"],
+              "n_connections": hdr["n_connections"]}
+    for f in ("score", "count", "peak_id", "x", "y"):
+        v = per[f].astype(np.float64)
+        arrays["person_" + f] = np.where(used.reshape(used.shape + (1,) * (v.ndim - 2)), v, 0.0)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float64))
 
 
 def run_ours(args):
@@ -242,7 +264,7 @@ def run_ours(args):
     # slot 1 runs on its own stream, so the tails and launch gaps of one batch's kernels are filled by the other's.
     # One batch is in flight when the timed region starts and the region ends with opb_stream_join, so K steps contain
     # K complete pipeline passes, K record downloads and (N > 1) K all-gathers.
-    res_state = {"slot": 0, "primed": False, "hdr": None}
+    res_state = {"slot": 0, "hdr": None, "per": None}
 
     def res_submit():
         sl = res_state["slot"]
@@ -253,12 +275,9 @@ def run_ours(args):
         res_state["slot"] ^= 1
 
     def step_resident():
-        if not res_state["primed"]:
-            res_submit()
-            res_state["primed"] = True
         res_submit()
-        hdr, per = eng.stream_collect(res_state["slot"])           # the batch submitted one step earlier (and its all-gather)
-        res_state["hdr"] = hdr
+        # the batch submitted one step earlier (and its all-gather)
+        res_state["hdr"], res_state["per"] = eng.stream_collect(res_state["slot"])
 
     def step_e2e_sync():
         eng._check(eng.lib.opb_detect_batch(eng.ctx, C.c_void_p(imgs_host.data_ptr()), native.OPB_HOST, B, H, W,
@@ -270,7 +289,7 @@ def run_ours(args):
     # memory on the copy stream, runs the pipeline and reads its records back; the upload of batch i+1 overlaps
     # the kernels of batch i.  One batch is in flight when the timed region starts and one when it ends, so K
     # steps contain exactly K uploads, K pipeline passes and K result downloads.
-    e2e_state = {"slot": 0, "primed": False, "hdr": None}
+    e2e_state = {"slot": 0, "hdr": None}
 
     def e2e_submit():
         sl = e2e_state["slot"]
@@ -281,13 +300,14 @@ def run_ours(args):
         e2e_state["slot"] ^= 1
 
     def step_e2e():
-        if not e2e_state["primed"]:
-            e2e_submit()
-            e2e_state["primed"] = True
         e2e_submit()                                               # batch i+1 goes up ...
         e2e_state["hdr"], _ = eng.stream_collect(e2e_state["slot"])   # ... while batch i finishes; read its records
 
-    def timed(fn, steps, warmup):
+    def timed(fn, steps, warmup, prime=None):
+        # `prime` puts the first batch in flight before the warm-up, so that with any --warmup (0 included) the timed
+        # region holds exactly `steps` submits
+        if prime is not None:
+            prime()
         for _ in range(warmup):
             fn()
         if world > 1:
@@ -316,9 +336,18 @@ def run_ours(args):
     sampler = ClockSampler(local_rank) if rank == 0 else None
     if sampler:
         sampler.start()
-    ms_total, launches = timed(step_resident, args.steps, args.warmup)
+    ms_total, launches = timed(step_resident, args.steps, args.warmup, prime=res_submit)
     per_rank_ms = [m / args.steps for m in timed.per_rank_ms]
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        if world > 1:   # the caller's view at N > 1: every rank's records, all-gathered with the last collected batch
+            g = gathered[res_state["slot"]].cpu().numpy().reshape(world, rec_bytes)
+            hb = B * native.HEADER_DTYPE.itemsize
+            hdr = np.concatenate([np.frombuffer(g[r, :hb].tobytes(), native.HEADER_DTYPE) for r in range(world)])
+            per = np.concatenate([np.frombuffer(g[r, hb:].tobytes(), native.PERSON_DTYPE).reshape(B, -1) for r in range(world)])
+        else:
+            hdr, per = res_state["hdr"], res_state["per"]
+        dump_records(args.dump_outputs, hdr, per)
     # correctness of the timed path: 8 persons per frame (last collected batch and the one still in flight)
     hdr_last, _ = eng.stream_collect(res_state["slot"] ^ 1)
     for hdr in (res_state["hdr"], hdr_last):
@@ -330,7 +359,7 @@ def run_ours(args):
             for r in range(world):
                 gh = np.frombuffer(g[r, :hdr_dev.numel()].tobytes(), native.HEADER_DTYPE)
                 assert (gh["status"] == 0).all() and (gh["n_persons"] == 8).all(), (r, gh)
-    ms_e2e, _ = timed(step_e2e, args.steps, args.warmup)
+    ms_e2e, _ = timed(step_e2e, args.steps, args.warmup, prime=e2e_submit)
     hdr_last, _ = eng.stream_collect(e2e_state["slot"] ^ 1)         # drain the batch still in flight
     for hh in (e2e_state["hdr"], hdr_last):
         assert (hh["status"] == 0).all() and (hh["n_persons"] == 8).all()
@@ -548,6 +577,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-stage-timing", action="store_true", help="skip the per-stage re-launches (clean ncu launch lists)")
     ap.add_argument("--no-parity-extra", action="store_true", help="skip the other-precision throughput extras (child processes)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the person records the timed path returned in its last step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -125,8 +125,8 @@ def test_camera_demo_import_flow_and_drawing():
 
 def test_demo_import_flow_face_hand_modules():
     """What demo.py does before inference (reference demo.py:1-20), flat imports: the three detector modules and
-    their drawing helpers; host-only helpers (draw_*, crop_face) checked against the reference's own functions when
-    the reference tree is present."""
+    their drawing helpers; host-only helpers (draw_*, crop_face) checked against the reference's own functions
+    (their digest in tests/golden/host_helpers_ref.json)."""
     import subprocess
     import sys
     code = (
@@ -153,16 +153,11 @@ def test_demo_import_flow_face_hand_modules():
     out = os.path.join(tempfile.mkdtemp(), "draw.npy")
     r = subprocess.run([sys.executable, "-c", code, out], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
     assert r.returncode == 0 and "ok" in r.stdout, r.stdout
-    from oracle import reference_loader
-    if reference_loader.available():
-        rf, rh = reference_loader.load_face(), reference_loader.load_hand()
-        img = np.zeros((100, 120, 3), np.uint8)
-        face = [[10 + i, 20 + (i % 7), np.float32(0.5)] if i % 5 else None for i in range(70)]
-        hand = [[15 + 3 * i, 30 + (i % 4), np.float32(0.5)] if i % 6 else None for i in range(21)]
-        pf, _ = rf.crop_face(np.arange(100 * 120 * 3, dtype=np.uint8).reshape(100, 120, 3), (30, 20, 40, 50))
-        ref = np.concatenate([rf.draw_face_keypoints(img, face, (3, 4)).ravel(),
-                              rh.draw_hand_keypoints(img, hand, (3, 4)).ravel(), pf.ravel()])
-        assert np.array_equal(np.load(out), ref)
+    import json
+    from conftest import GOLDEN
+    from oracle import make_goldens as MG
+    with open(os.path.join(GOLDEN, "host_helpers_ref.json")) as f:
+        assert MG.digest(np.load(out)) == json.load(f)["demo_face_hand_drawing"]
 
 
 

@@ -389,7 +389,7 @@ def test_precise_path_device_cubic_ingest(weights_model):
 
 @pytest.mark.parametrize("precision", ["parity", "comp"])
 def test_precise_path_480(weights_model, precision):
-    _check_precise(weights_model, precision, "precise_480_he0.npz", pkg("synthetic").procedural_image(480, 480, seed=3), 7)
+    _check_precise(weights_model, precision, "precise_480_he0.npz", pkg("synthetic").procedural_image(480, 480, seed=3), 9)
 
 
 @pytest.mark.parametrize("precision", ["parity", "comp"])

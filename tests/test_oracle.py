@@ -5,7 +5,18 @@ import numpy as np
 import pytest
 
 from conftest import load_golden, pkg, split_conns
+from oracle import make_goldens
 from oracle import restate as R
+
+
+@pytest.fixture(autouse=True)
+def golden_torch_threads():
+    """The torch-CPU convolutions run with the thread count the goldens were made with (their last bits depend on it)."""
+    import torch
+    saved = torch.get_num_threads()
+    torch.set_num_threads(make_goldens.TORCH_THREADS)
+    yield
+    torch.set_num_threads(saved)
 
 
 def test_layer_table_matches_package():
@@ -91,8 +102,8 @@ def test_precise_path_480(he_weights):
     g = load_golden("precise_480_he0.npz")
     img = pkg("synthetic").procedural_image(480, 480, seed=3)
     poses, scores, parts = R.detect_precise(he_weights, img, return_parts=True)
-    assert np.array_equal(parts["pafs"][:, ::7, ::7], g["pafs_sample"])
-    assert np.array_equal(parts["heatmaps"][:, ::7, ::7], g["heatmaps_sample"])
+    assert np.array_equal(parts["pafs"][:, ::9, ::9], g["pafs_sample"])
+    assert np.array_equal(parts["heatmaps"][:, ::9, ::9], g["heatmaps_sample"])
     assert np.array_equal(parts["all_peaks"], g["all_peaks"])
     assert np.array_equal(parts["subsets"], g["subsets"])
     assert np.array_equal(poses, g["poses"]) and np.array_equal(scores, g["scores"])

@@ -2,10 +2,9 @@
 (SciPy gaussian_filter, OpenCV resize) and against the reference's own helper on many random shapes -- the oracle is
 only as good as these restatements (SURVEY.md 8c: "parity unpinned" boundaries)."""
 import numpy as np
-import pytest
 from hypothesis import given, settings, strategies as st
 
-from oracle import reference_loader
+from conftest import load_golden
 from oracle import restate as R
 
 
@@ -26,14 +25,13 @@ def test_cv2_linear_u8_restatement_random_shapes(h0, w0, h, w, seed):
     assert np.array_equal(R.cv2_resize_linear_u8(img, (w, h)), cv2.resize(img, (w, h)))
 
 
-@pytest.mark.skipif(not reference_loader.available(), reason="reference tree not present")
-@settings(max_examples=200, deadline=None)
-@given(st.integers(16, 2000), st.integers(16, 2000), st.sampled_from([368, 320, 184, 552, 736]))
-def test_compute_optimal_size_matches_reference(h, w, size):
-    ref = reference_loader.load()
-    det = ref.PoseDetector.__new__(ref.PoseDetector)
-    img = np.zeros((h, w, 3), np.uint8)
-    assert tuple(R.compute_optimal_size(img, size)) == tuple(det.compute_optimal_size(img, size))
+def test_compute_optimal_size_matches_reference():
+    """The reference's own compute_optimal_size on the corners of the 16..2000 range and 4 000 seeded random
+    (h, w, size) triples (tests/golden/optimal_size_ref.npz, oracle/make_goldens.py host_helper_goldens)."""
+    g = load_golden("optimal_size_ref.npz")
+    for (h, w, size), want in zip(g["h_w_size"], g["optimal_size"]):
+        img = np.zeros((int(h), int(w), 3), np.uint8)
+        assert tuple(R.compute_optimal_size(img, int(size))) == tuple(want), (h, w, size)
 
 
 @settings(max_examples=25, deadline=None)
