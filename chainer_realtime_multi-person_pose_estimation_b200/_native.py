@@ -83,6 +83,8 @@ _SIGNATURES = {
                                        C.c_void_p, C.c_void_p, C.c_void_p]),
     "opb_keypoints_from_heatmaps": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                               C.c_double, C.c_void_p, C.c_void_p]),
+    "opb_keypoints_detect_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
+                                             C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]),
     "opb_precise_add_scale_unpadded": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                                  C.c_int, C.c_int]),
     "opb_get_image_detail": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.POINTER(C.c_int), C.c_void_p,
@@ -449,6 +451,31 @@ class Engine(object):
                                                   _ptr(maps) if return_maps else None))
         kps = self._keypoint_list(out, valid)
         return (kps, maps) if return_maps else kps
+
+    def keypoints_detect_batch(self, imgs, net_size, thresh, mirrors, return_maps=False):
+        """A list of BGR crops of any sizes -> one keypoint list per crop, as keypoints_detect returns it, from one
+        upload, one forward and one launch per post-process stage (opb_keypoints_detect_batch).  `mirrors`: one flag
+        for all crops or one per crop.  With return_maps, also the [C-1, h_i, w_i] maps of every crop."""
+        crops = [np.ascontiguousarray(a, np.uint8) for a in imgs]
+        n = len(crops)
+        mirror = np.array([bool(mirrors)] * n if np.ndim(mirrors) == 0 else [bool(m) for m in mirrors], np.int32)
+        if len(mirror) != n:
+            raise ValueError("%d mirror flags for %d crops" % (len(mirror), n))
+        dims = np.array([a.shape[:2] for a in crops], np.int32).reshape(n, 2)
+        packed = np.concatenate([a.ravel() for a in crops]) if n else np.zeros(0, np.uint8)
+        planes = self.kp_channels - 1
+        out = np.empty((n, planes, 3), np.float64)
+        valid = np.empty((n, planes), np.int32)
+        sizes = [planes * int(h) * int(w) for h, w in dims]
+        maps = np.empty(sum(sizes), np.float32) if return_maps else None
+        self._check(self.lib.opb_keypoints_detect_batch(self.ctx, _ptr(packed), OPB_HOST, n, _ptr(dims), _ptr(mirror),
+                                                        int(net_size), float(thresh), _ptr(out), _ptr(valid),
+                                                        _ptr(maps)))
+        kps = [self._keypoint_list(out[i], valid[i]) for i in range(n)]
+        if not return_maps:
+            return kps
+        ends = np.cumsum(sizes)
+        return kps, [maps[e - s:e].reshape(planes, int(h), int(w)) for e, s, (h, w) in zip(ends, sizes, dims)]
 
     def keypoints_from_heatmaps(self, heatmaps, thresh, mirror=False):
         """heatmaps [C,H,W] float32, background channel already dropped (opb_keypoints_from_heatmaps)."""

@@ -29,24 +29,50 @@ __device__ __forceinline__ void cv_linear_axis(int d, double scale, int src_n, b
   s1 = min(max(s + 1, 0), src_n - 1);
 }
 
-// src [n][h0][w0][3] uint8 -> dst [n][h][w][3] uint8; grid (ceil(w/32), ceil(h/8), n), block (32, 8)
-__global__ void __launch_bounds__(256)
-resize_linear_u8_kernel(const uint8_t* __restrict__ src, int h0, int w0, uint8_t* __restrict__ dst, int h, int w,
-                        double scale_x, double scale_y) {
-  const int x = blockIdx.x * 32 + threadIdx.x, y = blockIdx.y * 8 + threadIdx.y, n = blockIdx.z;
-  if (x >= w || y >= h) return;
+// One output pixel (x, y) of the INTER_LINEAR resize of the image img [h0][w0][3] into o[0..2].  With h0 == h and
+// w0 == w the arithmetic is the identity (f = 0: coefficients 2048 / 0), so no size needs a separate copy path.
+__device__ __forceinline__ void resize_linear_u8_pixel(const uint8_t* __restrict__ img, int h0, int w0, int x, int y,
+                                                       double scale_x, double scale_y, uint8_t* __restrict__ o) {
   int sx0, sx1, a0, a1, sy0, sy1, b0, b1;
   cv_linear_axis(x, scale_x, w0, true, sx0, sx1, a0, a1);
   cv_linear_axis(y, scale_y, h0, false, sy0, sy1, b0, b1);
-  const uint8_t* r0 = src + (static_cast<size_t>(n) * h0 + sy0) * w0 * 3;
-  const uint8_t* r1 = src + (static_cast<size_t>(n) * h0 + sy1) * w0 * 3;
-  uint8_t* o = dst + ((static_cast<size_t>(n) * h + y) * w + x) * 3;
+  const uint8_t* r0 = img + static_cast<size_t>(sy0) * w0 * 3;
+  const uint8_t* r1 = img + static_cast<size_t>(sy1) * w0 * 3;
 #pragma unroll
   for (int c = 0; c < 3; ++c) {
     const int d0 = r0[sx0 * 3 + c] * a0 + r0[sx1 * 3 + c] * a1;
     const int d1 = r1[sx0 * 3 + c] * a0 + r1[sx1 * 3 + c] * a1;
     o[c] = static_cast<uint8_t>((((b0 * (d0 >> 4)) >> 16) + ((b1 * (d1 >> 4)) >> 16) + 2) >> 2);
   }
+}
+
+// src [n][h0][w0][3] uint8 -> dst [n][h][w][3] uint8; grid (ceil(w/32), ceil(h/8), n), block (32, 8)
+__global__ void __launch_bounds__(256)
+resize_linear_u8_kernel(const uint8_t* __restrict__ src, int h0, int w0, uint8_t* __restrict__ dst, int h, int w,
+                        double scale_x, double scale_y) {
+  const int x = blockIdx.x * 32 + threadIdx.x, y = blockIdx.y * 8 + threadIdx.y, n = blockIdx.z;
+  if (x >= w || y >= h) return;
+  resize_linear_u8_pixel(src + static_cast<size_t>(n) * h0 * w0 * 3, h0, w0, x, y, scale_x, scale_y,
+                         dst + ((static_cast<size_t>(n) * h + y) * w + x) * 3);
+}
+
+// One crop of a ragged batch: crop i = h0 x w0 x 3 uint8 at byte offset `src_off` of the packed source.
+struct RaggedCrop {
+  long long src_off;
+  int h0, w0;
+  double scale_x, scale_y;   // 1 / (dst / src) in double, as cv2::resize forms them
+};
+
+// Crops of different sizes packed back to back -> dst [n][h][w][3] (one network-input slot per crop);
+// grid (ceil(w/32), ceil(h/8), n), block (32, 8).
+__global__ void __launch_bounds__(256)
+resize_linear_u8_ragged_kernel(const uint8_t* __restrict__ src, const RaggedCrop* __restrict__ crops,
+                               uint8_t* __restrict__ dst, int h, int w) {
+  const int x = blockIdx.x * 32 + threadIdx.x, y = blockIdx.y * 8 + threadIdx.y, n = blockIdx.z;
+  if (x >= w || y >= h) return;
+  const RaggedCrop c = crops[n];
+  resize_linear_u8_pixel(src + c.src_off, c.h0, c.w0, x, y, c.scale_x, c.scale_y,
+                         dst + ((static_cast<size_t>(n) * h + y) * w + x) * 3);
 }
 
 // ---- cv2.resize(orig_img, ..., interpolation=cv2.INTER_CUBIC) on uint8 BGR (detect_precise, pose_detector.py:443) ----

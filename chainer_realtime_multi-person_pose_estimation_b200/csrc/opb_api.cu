@@ -134,11 +134,13 @@ struct PostWs {           // post-process workspace for (N, map_h, map_w)
 
 struct KpWs {             // face / hand post-process workspace (grown on demand)
   size_t cap = 0;             // floats per buffer
-  int planes = 0;
-  float* up = nullptr;        // upsampled maps [planes][H][W]
+  int records = 0;
+  size_t stage_cap = 0;       // bytes of h_stage
+  float* up = nullptr;        // upsampled maps of every crop of a chunk, [planes][h_i][w_i] back to back
   float* tmp = nullptr;       // after the axis-0 pass
-  ChannelMax* res = nullptr;  // [planes]
+  ChannelMax* res = nullptr;  // [crops][planes]
   ChannelMax* h_res = nullptr;  // pinned
+  uint8_t* h_stage = nullptr;   // pinned: [crop tables | crops] of one upload
 };
 
 }  // namespace
@@ -1494,6 +1496,7 @@ void opb_destroy(opb_ctx* ctx) {
   if (ctx->ov_buf) cudaFree(ctx->ov_buf);
   if (ctx->kp_ws) {
     cudaFree(ctx->kp_ws->up); cudaFree(ctx->kp_ws->tmp); cudaFree(ctx->kp_ws->res); cudaFreeHost(ctx->kp_ws->h_res);
+    cudaFreeHost(ctx->kp_ws->h_stage);
     delete ctx->kp_ws;
   }
   for (auto& sl : ctx->slots) {
@@ -2569,84 +2572,194 @@ int opb_stream_collect(opb_ctx* ctx, int slot, opb_image_header* headers_out, op
   return OPB_OK;
 }
 
-static int kp_workspace(opb_ctx* ctx, int planes, int H, int W, KpWs** out) {
+// Face / hand nets on ragged batches: n crops of different sizes share one upload, one resize launch, one forward of
+// the chain for the next batch size in kKpBuckets, and one launch per post-process stage.
+static const int kKpBuckets[] = {1, 2, 4, 8, 16, 32};
+static const int kKpMaxCrops = 32;   // larger batches run in chunks of this many crops
+static const int kKpUpsamplePlanes = 19;   // planes per block of upsample_bilinear_ac_ragged_kernel
+
+static int kp_bucket(int n) {
+  for (int b : kKpBuckets)
+    if (b >= n) return b;
+  return kKpMaxCrops;
+}
+
+static size_t align256(size_t v) { return (v + 255) & ~size_t(255); }
+
+static int kp_workspace(opb_ctx* ctx, size_t floats, int records, size_t stage_bytes, KpWs** out) {
   if (!ctx->kp_ws) ctx->kp_ws = new KpWs();
   KpWs* ws = ctx->kp_ws;
-  const size_t need = static_cast<size_t>(planes) * H * W;
-  if (ws->cap < need || ws->planes < planes) {
+  if (ws->cap < floats || ws->records < records) {
     OPB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     cudaFree(ws->up); cudaFree(ws->tmp); cudaFree(ws->res); cudaFreeHost(ws->h_res);
-    ws->up = ws->tmp = nullptr; ws->res = nullptr; ws->h_res = nullptr; ws->cap = 0; ws->planes = 0;
-    OPB_CUDA(ctx, cudaMalloc(reinterpret_cast<void**>(&ws->up), need * 4));
-    OPB_CUDA(ctx, cudaMalloc(reinterpret_cast<void**>(&ws->tmp), need * 4));
-    OPB_CUDA(ctx, cudaMalloc(reinterpret_cast<void**>(&ws->res), sizeof(ChannelMax) * planes));
-    OPB_CUDA(ctx, cudaMallocHost(reinterpret_cast<void**>(&ws->h_res), sizeof(ChannelMax) * planes));
-    ws->cap = need; ws->planes = planes;
+    ws->up = ws->tmp = nullptr; ws->res = nullptr; ws->h_res = nullptr; ws->cap = 0; ws->records = 0;
+    OPB_CUDA(ctx, cudaMalloc(reinterpret_cast<void**>(&ws->up), floats * 4));
+    OPB_CUDA(ctx, cudaMalloc(reinterpret_cast<void**>(&ws->tmp), floats * 4));
+    OPB_CUDA(ctx, cudaMalloc(reinterpret_cast<void**>(&ws->res), sizeof(ChannelMax) * records));
+    OPB_CUDA(ctx, cudaMallocHost(reinterpret_cast<void**>(&ws->h_res), sizeof(ChannelMax) * records));
+    ws->cap = floats; ws->records = records;
+  }
+  if (ws->stage_cap < stage_bytes) {
+    OPB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    cudaFreeHost(ws->h_stage);
+    ws->h_stage = nullptr; ws->stage_cap = 0;
+    OPB_CUDA(ctx, cudaMallocHost(reinterpret_cast<void**>(&ws->h_stage), stage_bytes));
+    ws->stage_cap = stage_bytes;
   }
   *out = ws;
   return OPB_OK;
 }
 
-// smooth ws->up [planes][H][W] (both passes), per-plane maximum, records to the host
-static int kp_peaks(opb_ctx* ctx, KpWs* ws, int planes, int H, int W, int mirror, double thresh, double* out, int32_t* valid) {
-  dim3 block(32, 8), grid((W + 31) / 32, (H + 7) / 8, planes);
-  gauss_pass_kernel<0><<<grid, block, 0, ctx->stream>>>(ws->up, ws->tmp, H, W, ctx->taps);
-  gauss_pass_kernel<1><<<grid, block, 0, ctx->stream>>>(ws->tmp, ws->up, H, W, ctx->taps);
-  channel_argmax_kernel<<<planes, 256, 0, ctx->stream>>>(ws->up, H, W, mirror, ws->res);
+// Appends a crop of h x w maps to a ragged table: its place in the packed maps and its first block in the upsample
+// and per-plane launches.
+static void kp_add_crop(RaggedMaps& t, int h, int w, int mirror, int planes, long long& floats, int& blk_up,
+                        int& blk_plane) {
+  t.off = floats; t.h = h; t.w = w; t.mirror = mirror ? 1 : 0; t.pad_ = 0;
+  t.tiles_x = (w + 31) / 32;
+  t.tiles = t.tiles_x * ((h + 7) / 8);
+  t.blk_up = blk_up; t.blk_plane = blk_plane;
+  floats += static_cast<long long>(planes) * h * w;
+  blk_up += t.tiles * ((planes + kKpUpsamplePlanes - 1) / kKpUpsamplePlanes);
+  blk_plane += t.tiles * planes;
+}
+
+// Smooths ws->up (both passes) and takes the per-plane maximum of every crop of `tab` (d_tab: its device copy), then
+// one copy of all records to the host and one synchronise.  out [n][planes][3], valid [n][planes].
+static int kp_peaks(opb_ctx* ctx, KpWs* ws, int n, int planes, const RaggedMaps* tab, const RaggedMaps* d_tab,
+                    int blk_plane, double thresh, double* out, int32_t* valid) {
+  const dim3 block(32, 8);
+  gauss_pass_ragged_kernel<0><<<blk_plane, block, 0, ctx->stream>>>(ws->up, ws->tmp, d_tab, n, ctx->taps);
+  gauss_pass_ragged_kernel<1><<<blk_plane, block, 0, ctx->stream>>>(ws->tmp, ws->up, d_tab, n, ctx->taps);
+  channel_argmax_ragged_kernel<<<n * planes, 256, 0, ctx->stream>>>(ws->up, d_tab, planes, ws->res);
   ctx->launches += 3;
   OPB_CUDA(ctx, cudaGetLastError());
-  OPB_CUDA(ctx, cudaMemcpyAsync(ws->h_res, ws->res, sizeof(ChannelMax) * planes, cudaMemcpyDeviceToHost, ctx->stream));
+  OPB_CUDA(ctx, cudaMemcpyAsync(ws->h_res, ws->res, sizeof(ChannelMax) * n * planes, cudaMemcpyDeviceToHost, ctx->stream));
   OPB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   const float th = static_cast<float>(thresh);      // `max_value > thresh` with a float32 max_value compares in float32
-  for (int c = 0; c < planes; ++c) {
-    const ChannelMax& r = ws->h_res[c];
-    valid[c] = r.value > th ? 1 : 0;
-    // np.array(np.where(g == m)).flatten() = [y0..yk-1, x0..xk-1]; the reference reads [1] as x and [0] as y
-    const int y0 = r.key0 / W, x0 = r.key0 - y0 * W;
-    out[c * 3 + 0] = r.count >= 2 ? static_cast<double>(r.key1 / W) : static_cast<double>(x0);
-    out[c * 3 + 1] = static_cast<double>(y0);
-    out[c * 3 + 2] = static_cast<double>(r.value);
+  for (int i = 0; i < n; ++i) {
+    const int W = tab[i].w;
+    for (int c = i * planes; c < (i + 1) * planes; ++c) {
+      const ChannelMax& r = ws->h_res[c];
+      valid[c] = r.value > th ? 1 : 0;
+      // np.array(np.where(g == m)).flatten() = [y0..yk-1, x0..xk-1]; the reference reads [1] as x and [0] as y
+      const int y0 = r.key0 / W, x0 = r.key0 - y0 * W;
+      out[c * 3 + 0] = r.count >= 2 ? static_cast<double>(r.key1 / W) : static_cast<double>(x0);
+      out[c * 3 + 1] = static_cast<double>(y0);
+      out[c * 3 + 2] = static_cast<double>(r.value);
+    }
   }
   return OPB_OK;
+}
+
+// One chunk of at most kKpMaxCrops crops (arguments checked by the caller).
+static int kp_detect_chunk(opb_ctx* ctx, const uint8_t* imgs, int imgs_loc, int n, const int32_t* dims,
+                           const int32_t* mirror, int net, double thresh, double* out, int32_t* valid, float* maps_out) {
+  const int planes = ctx->kp_out - 1;              // the last channel is background (face_detector.py:59)
+  const int bucket = kp_bucket(n), lo = net / 8;
+  Chain* ch = nullptr;
+  int rc = get_chain(ctx, bucket, net, net, &ch);
+  if (rc) return rc;
+  std::vector<RaggedCrop> rz(n);
+  std::vector<RaggedMaps> tab(n);
+  size_t crop_bytes = 0;
+  long long floats = 0;
+  int blk_up = 0, blk_plane = 0;
+  for (int i = 0; i < n; ++i) {
+    const int h = dims[2 * i], w = dims[2 * i + 1];
+    rz[i].src_off = static_cast<long long>(crop_bytes);
+    rz[i].h0 = h; rz[i].w0 = w;
+    rz[i].scale_x = 1.0 / (static_cast<double>(net) / w);   // cv2::resize: scale = 1 / (dsize / ssize)
+    rz[i].scale_y = 1.0 / (static_cast<double>(net) / h);
+    crop_bytes += static_cast<size_t>(h) * w * 3;
+    kp_add_crop(tab[i], h, w, mirror[i], planes, floats, blk_up, blk_plane);
+  }
+  // one upload: [resize table | post-process table | crops (host input only)]
+  const size_t off_tab = align256(sizeof(RaggedCrop) * n), off_img = align256(off_tab + sizeof(RaggedMaps) * n);
+  const size_t up_bytes = imgs_loc == OPB_HOST ? off_img + crop_bytes : off_tab + sizeof(RaggedMaps) * n;
+  KpWs* ws = nullptr;
+  if ((rc = kp_workspace(ctx, static_cast<size_t>(floats), n * planes, up_bytes, &ws))) return rc;
+  if ((rc = ensure_ingest(ctx, up_bytes))) return rc;
+  memcpy(ws->h_stage, rz.data(), sizeof(RaggedCrop) * n);
+  memcpy(ws->h_stage + off_tab, tab.data(), sizeof(RaggedMaps) * n);
+  if (imgs_loc == OPB_HOST) memcpy(ws->h_stage + off_img, imgs, crop_bytes);
+  OPB_CUDA(ctx, cudaMemcpyAsync(ctx->ingest_buf, ws->h_stage, up_bytes, cudaMemcpyHostToDevice, ctx->stream));
+  const uint8_t* d_src = imgs_loc == OPB_HOST ? ctx->ingest_buf + off_img : imgs;
+  const RaggedCrop* d_rz = reinterpret_cast<const RaggedCrop*>(ctx->ingest_buf);
+  const RaggedMaps* d_tab = reinterpret_cast<const RaggedMaps*>(ctx->ingest_buf + off_tab);
+  // slots past the last crop are zeroed; the network computes every image of the batch independently, and nothing
+  // after it reads those slots
+  const size_t slot_bytes = static_cast<size_t>(net) * net * 3;
+  if (bucket > n) OPB_CUDA(ctx, cudaMemsetAsync(ch->img_u8 + n * slot_bytes, 0, (bucket - n) * slot_bytes, ctx->stream));
+  // cv2.resize(crop, (368, 368)) (face_detector.py:31) of every crop, bit-exact uint8 INTER_LINEAR
+  resize_linear_u8_ragged_kernel<<<dim3((net + 31) / 32, (net + 7) / 8, n), dim3(32, 8), 0, ctx->stream>>>(
+      d_src, d_rz, ch->img_u8, net, net);
+  ctx->launches++;
+  OPB_CUDA(ctx, cudaGetLastError());
+  ch->img_u8_src = nullptr;
+  if ((rc = run_chain(ctx, ch, true))) return rc;
+  // F.resize_images(hs[-1], (crop_h, crop_w)) (face_detector.py:38) of every crop
+  upsample_bilinear_ac_ragged_kernel<<<blk_up, dim3(32, 8), 0, ctx->stream>>>(
+      ch->heat_lo, static_cast<long long>(ctx->kp_out) * lo * lo, planes, lo, lo, d_tab, n, ws->up, kKpUpsamplePlanes);
+  ctx->launches++;
+  OPB_CUDA(ctx, cudaGetLastError());
+  if (maps_out && (rc = copy_out(ctx, maps_out, ws->up, static_cast<size_t>(floats) * 4, OPB_HOST))) return rc;
+  return kp_peaks(ctx, ws, n, planes, tab.data(), d_tab, blk_plane, thresh, out, valid);
 }
 
 int opb_keypoints_from_heatmaps(opb_ctx* ctx, const float* heat, int heat_loc, int planes, int h, int w, int mirror,
                                 double thresh, double* out, int32_t* valid) {
   if (!ctx || !heat || !out || !valid || planes <= 0 || h <= 0 || w <= 0) return OPB_ERR_ARG;
   cudaSetDevice(ctx->device);
+  RaggedMaps tab;
+  long long floats = 0;
+  int blk_up = 0, blk_plane = 0;
+  kp_add_crop(tab, h, w, mirror, planes, floats, blk_up, blk_plane);
   KpWs* ws = nullptr;
-  int rc = kp_workspace(ctx, planes, h, w, &ws);
+  int rc = kp_workspace(ctx, static_cast<size_t>(floats), planes, sizeof(tab), &ws);
   if (rc) return rc;
-  if ((rc = copy_in(ctx, ws->up, heat, static_cast<size_t>(planes) * h * w * 4, heat_loc))) return rc;
-  return kp_peaks(ctx, ws, planes, h, w, mirror, thresh, out, valid);
+  if ((rc = ensure_ingest(ctx, sizeof(tab)))) return rc;
+  memcpy(ws->h_stage, &tab, sizeof(tab));
+  OPB_CUDA(ctx, cudaMemcpyAsync(ctx->ingest_buf, ws->h_stage, sizeof(tab), cudaMemcpyHostToDevice, ctx->stream));
+  if ((rc = copy_in(ctx, ws->up, heat, static_cast<size_t>(floats) * 4, heat_loc))) return rc;
+  return kp_peaks(ctx, ws, 1, planes, &tab, reinterpret_cast<const RaggedMaps*>(ctx->ingest_buf), blk_plane, thresh,
+                  out, valid);
+}
+
+int opb_keypoints_detect_batch(opb_ctx* ctx, const uint8_t* imgs, int imgs_loc, int n, const int32_t* dims,
+                               const int32_t* mirror, int net_size, double thresh, double* out, int32_t* valid,
+                               float* maps_out) {
+  if (!ctx) return OPB_ERR_ARG;
+  if (n < 0) OPB_FAIL(ctx, OPB_ERR_ARG, "opb_keypoints_detect_batch: n = " + std::to_string(n) + " < 0");
+  if (!ctx->kp_out) OPB_FAIL(ctx, OPB_ERR_STATE, "this context holds the pose net: load FaceNet / HandNet weights first");
+  if (n == 0) return OPB_OK;
+  if (!imgs || !dims || !mirror || !out || !valid) OPB_FAIL(ctx, OPB_ERR_ARG, "opb_keypoints_detect_batch: null argument");
+  if (net_size <= 0 || net_size % 8) OPB_FAIL(ctx, OPB_ERR_ARG, "net_size must be a positive multiple of 8");
+  for (int i = 0; i < n; ++i)
+    if (dims[2 * i] <= 0 || dims[2 * i + 1] <= 0)
+      OPB_FAIL(ctx, OPB_ERR_ARG, "crop " + std::to_string(i) + " has size " + std::to_string(dims[2 * i]) + "x" +
+                                     std::to_string(dims[2 * i + 1]));
+  cudaSetDevice(ctx->device);
+  const int planes = ctx->kp_out - 1;
+  for (int c0 = 0; c0 < n; c0 += kKpMaxCrops) {
+    const int m = std::min(n - c0, kKpMaxCrops);
+    int rc = kp_detect_chunk(ctx, imgs, imgs_loc, m, dims + 2 * c0, mirror + c0, net_size, thresh,
+                             out + static_cast<size_t>(c0) * planes * 3, valid + static_cast<size_t>(c0) * planes,
+                             maps_out);
+    if (rc) return rc;
+    for (int i = c0; i < c0 + m; ++i) {
+      const size_t px = static_cast<size_t>(dims[2 * i]) * dims[2 * i + 1];
+      imgs += px * 3;
+      if (maps_out) maps_out += px * planes;
+    }
+  }
+  return OPB_OK;
 }
 
 int opb_keypoints_detect(opb_ctx* ctx, const uint8_t* img, int img_loc, int img_h, int img_w, int net_size, int mirror,
                          double thresh, double* out, int32_t* valid, float* maps_out) {
   if (!ctx || !img || !out || !valid || img_h <= 0 || img_w <= 0) return OPB_ERR_ARG;
-  if (!ctx->kp_out) OPB_FAIL(ctx, OPB_ERR_STATE, "this context holds the pose net: load FaceNet / HandNet weights first");
-  cudaSetDevice(ctx->device);
-  Chain* ch = nullptr;
-  int rc = get_chain(ctx, 1, net_size, net_size, &ch);
-  if (rc) return rc;
-  const size_t in_b = static_cast<size_t>(img_h) * img_w * 3;
-  const uint8_t* d_src = img;
-  if (img_loc == OPB_HOST) {
-    if ((rc = ensure_ingest(ctx, in_b + 512))) return rc;
-    if ((rc = copy_in(ctx, ctx->ingest_buf, img, in_b, OPB_HOST))) return rc;
-    d_src = ctx->ingest_buf;
-  }
-  // cv2.resize(crop, (368, 368)) (face_detector.py:31), bit-exact uint8 INTER_LINEAR on the device
-  if ((rc = launch_resize_u8(ctx, d_src, 1, img_h, img_w, ch->img_u8, net_size, net_size))) return rc;
-  ch->img_u8_src = nullptr;
-  if ((rc = run_chain(ctx, ch, true))) return rc;
-  const int planes = ctx->kp_out - 1;              // the last channel is background (face_detector.py:59)
-  KpWs* ws = nullptr;
-  if ((rc = kp_workspace(ctx, planes, img_h, img_w, &ws))) return rc;
-  // F.resize_images(hs[-1], (crop_h, crop_w)) (face_detector.py:38)
-  if ((rc = launch_upsample(ctx, ch->heat_lo, planes, net_size / 8, net_size / 8, ws->up, img_h, img_w))) return rc;
-  if (maps_out && (rc = copy_out(ctx, maps_out, ws->up, static_cast<size_t>(planes) * img_h * img_w * 4, OPB_HOST))) return rc;
-  return kp_peaks(ctx, ws, planes, img_h, img_w, mirror, thresh, out, valid);
+  const int32_t dims[2] = {img_h, img_w}, mir[1] = {mirror};
+  return opb_keypoints_detect_batch(ctx, img, img_loc, 1, dims, mir, net_size, thresh, out, valid, maps_out);
 }
 
 void* opb_device_buffer(opb_ctx* ctx, int which) {
@@ -2661,6 +2774,7 @@ void* opb_device_buffer(opb_ctx* ctx, int which) {
     case 4: return ws ? ws->headers : nullptr;
     case 5: return ws ? ws->persons : nullptr;
     case 6: return ws ? ws->peaks : nullptr;
+    case 7: return ch ? ch->img_u8 : nullptr;
     default: return nullptr;
   }
 }

@@ -225,6 +225,57 @@ __device__ __forceinline__ float ac_sample(const float* __restrict__ plane, int 
   return r;
 }
 
+// ---- ragged batches: crops of different sizes in one launch -------------------------------------
+// Crop i's full-resolution maps are [planes][h][w] floats at `off` of one packed buffer.  A launch covers every crop
+// with a flat block index: the crop's blocks start at blk_up (upsample: plane groups x 32x8 tiles) or at blk_plane
+// (one block per plane and 32x8 tile: the Gaussian passes); ragged_crop_of finds the crop of a block.
+struct RaggedMaps {
+  long long off;      // float offset of the crop's first plane in the packed buffer
+  int h, w;
+  int tiles_x, tiles; // ceil(w/32), ceil(w/32) * ceil(h/8)
+  int blk_up;         // first block of the crop in upsample_bilinear_ac_ragged_kernel
+  int blk_plane;      // first block of the crop in the per-plane-tile launches
+  int mirror;         // keypoints: report positions in the horizontally flipped maps
+  int pad_;
+};
+
+// the last crop whose first block (blk_up or blk_plane) is <= b
+__device__ __forceinline__ int ragged_crop_of(const RaggedMaps* __restrict__ c, int n, int b, bool up) {
+  int lo = 0, hi = n - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if ((up ? c[mid].blk_up : c[mid].blk_plane) <= b) lo = mid;
+    else hi = mid - 1;
+  }
+  return lo;
+}
+
+// F.resize_images of every crop's low-resolution maps: in = slot i at in + i * in_stride ([planes][h][w] of it are
+// read), out = crop i's [planes][crops[i].h][crops[i].w] at crops[i].off.  Same operations in the same order as
+// upsample_bilinear_ac_kernel (ac_axis_frac / ac_tap / ac_sample), so the same bits.  Block (32, 8); one block =
+// one 32x8 tile of `planes_per_block` planes.
+__global__ void __launch_bounds__(256)
+upsample_bilinear_ac_ragged_kernel(const float* __restrict__ in, long long in_stride, int planes, int h, int w,
+                                   const RaggedMaps* __restrict__ crops, int n, float* __restrict__ out,
+                                   int planes_per_block) {
+  const int i = ragged_crop_of(crops, n, blockIdx.x, true);
+  const RaggedMaps c = crops[i];
+  const int local = blockIdx.x - c.blk_up, group = local / c.tiles, tile = local - group * c.tiles;
+  const int ty = tile / c.tiles_x, tx = tile - ty * c.tiles_x;
+  const int x = tx * 32 + threadIdx.x, y = ty * 8 + threadIdx.y;
+  if (x >= c.w || y >= c.h) return;
+  const AcTap t = ac_tap(ac_axis_frac(x, w, c.w, ac_step(w, c.w)), ac_axis_frac(y, h, c.h, ac_step(h, c.h)), w);
+  const int p_begin = group * planes_per_block, p_end = min(planes, p_begin + planes_per_block);
+  const size_t in_plane = static_cast<size_t>(h) * w, out_plane = static_cast<size_t>(c.h) * c.w;
+  const float* src = in + i * in_stride + p_begin * in_plane;
+  float* dst = out + c.off + p_begin * out_plane + static_cast<size_t>(y) * c.w + x;
+  for (int p = p_begin; p < p_end; ++p) {
+    __stcs(dst, ac_sample(src, w, t));
+    src += in_plane;
+    dst += out_plane;
+  }
+}
+
 // ---- cv2 INTER_CUBIC for float32 (A = -0.75), separable, replicate border ------------------
 __device__ __forceinline__ void cubic_taps(float t, float (&c)[4]) {
   const float A = -0.75f;

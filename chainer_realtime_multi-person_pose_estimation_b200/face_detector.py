@@ -42,6 +42,11 @@ class FaceDetector(object):
         return self.engine.keypoints_detect(face_img, params["face_inference_img_size"],
                                             params['face_heatmap_peak_thresh'])
 
+    def detect_batch(self, face_imgs):
+        """[self(img) for img in face_imgs], computed as one batch (opb_keypoints_detect_batch)."""
+        return self.engine.keypoints_detect_batch(face_imgs, params["face_inference_img_size"],
+                                                  params['face_heatmap_peak_thresh'], False)
+
     def create_gaussian_kernel(self, sigma=1, ksize=5):
         """The 2-D kernel of the reference's GPU branch (face_detector.py:44-52); kept for API compatibility --
         peak extraction here follows the CPU branch (scipy gaussian_filter) exactly."""

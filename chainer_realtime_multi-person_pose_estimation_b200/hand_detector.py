@@ -46,6 +46,18 @@ class HandDetector(object):
         return self.engine.keypoints_detect(hand_img, params["hand_inference_img_size"],
                                             params['hand_heatmap_peak_thresh'], mirror=left)
 
+    def detect_batch(self, hand_imgs, hand_types="right"):
+        """[self(img, hand_type=t) for img, t in zip(hand_imgs, hand_types)], computed as one batch
+        (opb_keypoints_detect_batch).  hand_types: one string for every crop, or one per crop; left crops are flipped
+        here and reported in the flipped maps' coordinates, as __call__ does."""
+        types = [hand_types] * len(hand_imgs) if isinstance(hand_types, str) else list(hand_types)
+        if len(types) != len(hand_imgs):
+            raise ValueError("%d hand types for %d crops" % (len(types), len(hand_imgs)))
+        left = [t == "left" for t in types]
+        crops = [cv2.flip(img, 1) if lf else img for img, lf in zip(hand_imgs, left)]
+        return self.engine.keypoints_detect_batch(crops, params["hand_inference_img_size"],
+                                                  params['hand_heatmap_peak_thresh'], left)
+
     def create_gaussian_kernel(self, sigma=1, ksize=5):
         """The 2-D kernel of the reference's GPU branch (hand_detector.py:44-52); kept for API compatibility --
         peak extraction here follows the CPU branch (scipy gaussian_filter) exactly."""

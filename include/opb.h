@@ -254,10 +254,24 @@ int opb_keypoints_detect(opb_ctx* ctx, const uint8_t* img, int img_loc, int img_
                          int mirror, double thresh, double* out, int32_t* valid, float* maps_out);
 int opb_keypoints_from_heatmaps(opb_ctx* ctx, const float* heat, int heat_loc, int planes, int h, int w,
                                 int mirror, double thresh, double* out, int32_t* valid);
+/* FaceDetector / HandDetector __call__ for n crops of different sizes in one pass.  imgs: crops packed back to back
+ * (crop i = dims[2i] x dims[2i+1] x 3 uint8 BGR at byte offset sum_{j<i} h_j*w_j*3), host or device; mirror[i] as in
+ * opb_keypoints_detect.  out [n][C-1][3], valid [n][C-1]; maps_out (host, may be NULL): the unsmoothed upsampled maps
+ * of every crop back to back ([C-1][h_i][w_i] each).
+ * One upload, one resize launch, one forward and one launch per post-process stage per chunk: the network runs at the
+ * next batch size of 1, 2, 4, 8, 16, 32 (the slots past the last crop hold zeros and are not post-processed), and
+ * n > 32 runs in chunks of 32 crops, each ending in one copy of the records to the host and one synchronise.
+ * Arguments are checked before anything is launched: n < 0, a NULL array or a crop side <= 0 -> OPB_ERR_ARG (the
+ * message names the crop); a pose-net context -> OPB_ERR_STATE; n == 0 -> OPB_OK.  opb_keypoints_detect is the
+ * n = 1 case of this call.                                                                                        */
+int opb_keypoints_detect_batch(opb_ctx* ctx, const uint8_t* imgs, int imgs_loc, int n, const int32_t* dims,
+                               const int32_t* mirror, int net_size, double thresh, double* out, int32_t* valid,
+                               float* maps_out);
 
 /* device pointers of the last opb_detect_batch outputs/intermediates (valid until the next
  * call with a different shape): 0 paf_lo, 1 heat_lo, 2 pafs (full-res), 3 heatmaps (full-res),
- * 4 headers, 5 persons, 6 peak table ([N,max_peaks] of {int32 type,x,y; float score})       */
+ * 4 headers, 5 persons, 6 peak table ([N,max_peaks] of {int32 type,x,y; float score}),
+ * 7 uint8 network input [N][H][W][3] of the last chain (the resized crops of opb_keypoints_detect_batch)       */
 void* opb_device_buffer(opb_ctx* ctx, int which);
 
 /* Detail of image `img` of the last opb_detect_batch / opb_precise_finish: the peak table
